@@ -131,6 +131,30 @@ def model_kwargs(name: str):
     return kw
 
 
+DUMP_PARAM_SAMPLE = 1 << 22      # --dump-outputs: a larger parameter vector is sampled down to this many elements (16 MB of float32)
+
+
+def dump_outputs(out_dir: str, trainer) -> None:
+    """Write what ``trainer.step()`` hands its caller once the last timed step's round has landed, as float32 ``.npy`` files:
+    ``loss`` (the last micro-batch's loss as read by the host) and ``params`` (the flat weight vector the model reads; above
+    DUMP_PARAM_SAMPLE elements, the elements at a fixed sorted sample of indices drawn with seed 0).
+
+    ACCO accumulates extra micro-batches while a round is still running, so how many ran depends on timing, and so do the inputs
+    the last step saw.  ``micro_batches`` (this rank's, whole run) and ``count_grad_tot`` (committed gradients, all ranks) are
+    written too, as float64: two dumps are comparable output for output only when these agree."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    params = trainer.params.detach()
+    if params.numel() > DUMP_PARAM_SAMPLE:
+        idx = torch.randint(params.numel(), (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        params = params[idx.to(params.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), trainer.loss_host.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params.npy"), params.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "micro_batches.npy"), np.array([trainer.micro_batches], dtype=np.float64))
+    np.save(os.path.join(out_dir, "count_grad_tot.npy"), np.array([trainer.sched.count_grad_tot], dtype=np.float64))
+
+
 def run_ours(a) -> dict:
     import torch
     import torch.distributed as dist
@@ -232,6 +256,8 @@ def run_ours(a) -> dict:
         loss = float(trainer.loss_host.item())
         n_params = trainer.len_params
         trainer._drain()
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, trainer)
     finally:
         os.chdir(cwd)
     tok = a.batch * a.seq
@@ -304,7 +330,7 @@ def run_reference_arm(a) -> dict:
 def main():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=20)
+    p.add_argument("--steps", type=int, default=20, help="timed steps (round flips) in each of the two timed passes")
     p.add_argument("--warmup", type=int, default=5)
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--model", default="llama125m")
@@ -321,7 +347,16 @@ def main():
     p.add_argument("--slow-ms", dest="slow_ms", type=float, default=0.0, help="extra GPU milliseconds per micro-batch on the slow rank")
     p.add_argument("--preset", default=None, choices=sorted(PRESETS_BENCH),
                    help="named BASELINE.json configurations (override --model/--batch/--seq/--n-acc/--method)")
+    p.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                   help="after the timed steps, write the last step's loss and weights (sampled) and the micro-batch / gradient "
+                        "counts that decide whether two dumps are comparable to DIR/*.npy (rank 0)")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs:
+        if a.impl == "reference":
+            p.error("--dump-outputs applies to --impl ours")
+        a.dump_outputs = os.path.abspath(a.dump_outputs)    # run_ours() works in a temporary directory
     if a.preset:
         for k, v in PRESETS_BENCH[a.preset].items():
             setattr(a, k, v)

@@ -28,6 +28,29 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip_multi)
 
 
+def _drop_process_group():
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized():
+        dist.destroy_process_group()
+
+
+@pytest.fixture(autouse=True)
+def _cpu_unless_marked_gpu(request, monkeypatch):
+    """Tests not marked `gpu` check the CPU / gloo paths.  The trainer, main.py and the launcher take CUDA whenever it is
+    available, so on a machine with a GPU these tests see none (the ranks they start set CUDA_VISIBLE_DEVICES="" themselves:
+    setting it here would leave torch's device count cached at 0 for the `gpu` tests).  The launcher also reuses an initialised
+    default process group, so these tests start and end without one: a `gpu` test's NCCL group is no group for CPU tensors,
+    and theirs is none for CUDA tensors."""
+    if "gpu" in request.keywords:
+        yield
+        return
+    import torch
+    _drop_process_group()
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
+    yield
+    _drop_process_group()
+
+
 @pytest.fixture
 def workdir(tmp_path, monkeypatch):
     """Run inside a scratch cwd: the trainer writes tensorboard/, checkpoints/, results.csv there."""

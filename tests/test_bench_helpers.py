@@ -1,7 +1,9 @@
-"""Host-side helpers of bench.py / tools (no GPU needed)."""
+"""Host-side helpers of bench.py / tools (no GPU needed), and one end-to-end `bench.py --dump-outputs` run on the GPU."""
 import importlib.util
 import os
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -53,6 +55,47 @@ def test_reference_arm_reports_unavailable_instead_of_crashing(monkeypatch, caps
     out = bench.run_reference_arm(args)
     assert out["impl"] == "reference"
     assert "unavailable" in out or "value" in out
+
+
+def test_dump_outputs_writes_loss_and_sampled_params(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs DIR`: float32 loss and weights; a vector above the cap is sampled the same way on every call."""
+    import numpy as np
+    import torch
+    bench = _load(os.path.join(ROOT, "bench.py"), "bench_mod4")
+    monkeypatch.setattr(bench, "DUMP_PARAM_SAMPLE", 1000)
+    sched = type("S", (), dict(count_grad_tot=7))()
+    small = type("T", (), dict(params=torch.randn(1000).bfloat16(), loss_host=torch.tensor([2.5]), micro_batches=9, sched=sched))()
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    loss, params = np.load(tmp_path / "small" / "loss.npy"), np.load(tmp_path / "small" / "params.npy")
+    assert loss.dtype == np.float32 and loss.tolist() == [2.5]
+    assert params.dtype == np.float32 and np.array_equal(params, small.params.float().numpy())
+    for name, want in (("micro_batches", 9), ("count_grad_tot", 7)):        # whether two dumps took the same schedule
+        got = np.load(tmp_path / "small" / f"{name}.npy")
+        assert got.dtype == np.float64 and got.tolist() == [want]
+    big = type("T", (), dict(params=torch.arange(5000, dtype=torch.float32), loss_host=torch.tensor([1.0]), micro_batches=9, sched=sched))()
+    bench.dump_outputs(str(tmp_path / "a"), big)
+    bench.dump_outputs(str(tmp_path / "b"), big)
+    a, b = np.load(tmp_path / "a" / "params.npy"), np.load(tmp_path / "b" / "params.npy")
+    assert a.shape == (1000,) and np.array_equal(a, b)
+    assert np.all(np.diff(a) >= 0) and a.min() >= 0 and a.max() < 5000     # sorted indices into the vector
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_on_the_gpu(tmp_path):
+    """`bench.py --steps 1 --dump-outputs DIR` end to end: DIR relative to the caller's cwd (the benchmark itself runs in a temporary
+    directory), one timed step, and finite float arrays written after it."""
+    import json
+    import subprocess
+    import numpy as np
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1", "--batch", "1", "--seq", "256",
+                        "--dump-outputs", "dump"], cwd=tmp_path, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
+    assert p.returncode == 0, p.stdout[-3000:]
+    res = json.loads([ln for ln in p.stdout.splitlines() if ln.startswith("{")][-1])
+    assert res["steps"] == 1
+    got = {n: np.load(tmp_path / "dump" / f"{n}.npy") for n in ("loss", "params", "micro_batches", "count_grad_tot")}
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in got.values())
+    assert got["params"].shape == (1 << 22,) and got["loss"].shape == (1,)
+    assert got["micro_batches"][0] >= res["config"]["micro_batches_timed"] and got["count_grad_tot"][0] >= 1
 
 
 def test_launch_summary_parses_ncu_csv(tmp_path, capsys):

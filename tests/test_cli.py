@@ -30,8 +30,7 @@ def test_shim_import():
     import trainer_decoupled as td
     import decoupled_trainer as dt
     import importlib.util
-    # by file path: the golden-trace test imports the REFERENCE's trainer_decoupled, which registers the reference's own `trainer_base` in
-    # sys.modules for the rest of the process
+    # by file path: this repo's shim, whatever module another import may have registered as `trainer_base` in sys.modules
     spec = importlib.util.spec_from_file_location("trainer_base_shim", os.path.join(ROOT, "trainer_base.py"))
     tb = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(tb)

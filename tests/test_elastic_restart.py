@@ -13,7 +13,7 @@ def clean_env(**extra):
     and that port is held by this very process)."""
     drop = ("MASTER_ADDR", "MASTER_PORT", "RANK", "WORLD_SIZE", "LOCAL_RANK", "LOCAL_WORLD_SIZE", "GROUP_RANK")
     env = {k: v for k, v in os.environ.items() if k not in drop and not k.startswith(("SLURM_", "TORCHELASTIC_"))}
-    env.update(OMP_NUM_THREADS="2", PYTHONPATH=ROOT, **extra)
+    env.update(OMP_NUM_THREADS="2", PYTHONPATH=ROOT, CUDA_VISIBLE_DEVICES="", **extra)     # CPU ranks even where a GPU is present
     return env
 
 

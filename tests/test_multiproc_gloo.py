@@ -11,9 +11,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _worker(rank, world, port, method, tmp, extra, q):
+    # every worker hides the GPUs before touching CUDA: these are CPU ranks, and the trainer takes CUDA whenever it sees a device
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank))
     os.chdir(tmp)
     torch.set_num_threads(2)
     from acco_b200 import DecoupledTrainer
@@ -92,7 +94,8 @@ def test_init_avg_mode_matches_reference_behaviour():
 def _worker3(rank, world, port, tmp, q):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank))
     os.chdir(tmp)
     torch.set_num_threads(1)
     from acco_b200 import DecoupledTrainer
@@ -138,8 +141,8 @@ def test_three_ranks_ragged_slices_all_methods_and_torch_ddp():
 def _worker_resume(rank, world, port, tmp, phase, q):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank),
-                      ACCO_RUN_ID="resume")
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank), ACCO_RUN_ID="resume")
     os.chdir(tmp)
     torch.set_num_threads(2)
     from acco_b200 import DecoupledTrainer
@@ -209,8 +212,8 @@ def test_two_rank_resume_restores_every_ranks_optimizer_shard():
 def _worker_preempt(rank, world, port, tmp, q):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank),
-                      ACCO_RUN_ID="pre")
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank), ACCO_RUN_ID="pre")
     os.chdir(tmp)
     torch.set_num_threads(2)
     from acco_b200 import DecoupledTrainer
@@ -256,7 +259,8 @@ def test_preemption_signal_on_one_rank_stops_every_rank_after_the_same_round():
 def _worker_dist_utils(rank, world, port, tmp, q):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), ACCO_RUN_ID="du")
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank), ACCO_RUN_ID="du")
     os.chdir(tmp)
     torch.set_num_threads(2)
     from acco_b200 import DecoupledTrainer

@@ -1,8 +1,8 @@
 import csv
 import os
-import sys
 import types
 
+import numpy as np
 import pytest
 import torch
 
@@ -11,6 +11,8 @@ from acco_b200.data import synthetic_pretrain_dataset, synthetic_sft_dataset, By
 from acco_b200.launch import DistEnv
 
 from helpers import LOG, ToyQuadratic, base_args, tiny_model
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def make(method="acco", model=None, ds=None, **kw):
@@ -94,67 +96,17 @@ def test_acco_equals_large_batch_ddp_when_estimate_is_exact(workdir):
     assert torch.equal(ta.model.w.detach(), td.model.w.detach())
 
 
-def _reference_available():
-    return os.path.isdir("/root/reference") and os.path.isfile("/root/reference/trainer_decoupled.py")
-
-
-def _import_reference_steps():
-    """Import the reference's step primitives with a stubbed omegaconf (not installed here)."""
-    if "omegaconf" not in sys.modules:
-        m = types.ModuleType("omegaconf")
-        m.OmegaConf = type("OmegaConf", (), {"to_container": staticmethod(lambda c, resolve=True: dict(c))})
-        sys.modules["omegaconf"] = m
-    # load by file path under a private name: `trainer_decoupled` may already be this repo's compatibility shim
-    import importlib.util
-    sys.path.insert(0, "/root/reference")
-    try:
-        spec = importlib.util.spec_from_file_location("_reference_trainer_decoupled", "/root/reference/trainer_decoupled.py")
-        ref = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref)
-    finally:
-        sys.path.remove("/root/reference")
-    return ref
-
-
-@pytest.mark.skipif(not _reference_available(), reason="reference checkout not mounted")
 def test_golden_trace_against_reference_step_functions(workdir):
-    """T1(a): drive the reference's own communication_step / update_buffers_step (CPU, gloo W=1,
-    AdamW(capturable=False)) and our trainer on the same toy; parameters after every flip must agree."""
-    import torch.distributed as dist
-    from acco_b200.launch import free_port
-    ref = _import_reference_steps()
-    os.environ["MASTER_ADDR"], os.environ["MASTER_PORT"] = "127.0.0.1", str(free_port())
-    if not dist.is_initialized():
-        dist.init_process_group("gloo", rank=0, world_size=1)
+    """T1(a): our trainer against the trace of the original ACCO implementation on the same toy, stored in
+    `golden/acco_reference_trace.npy` (float32, one row of parameters per flip).  The trace was produced by the original's own
+    `communication_step` / `update_buffers_step` (CPU, gloo W=1, AdamW(capturable=False), lr 0.1, betas (0.9, 0.95), no weight
+    decay, constant LR) from p0 = [1, 2, 3, 4] with gradient 0.1*(k+1)*p at the k-th evaluation: g0 at p0 fills the first
+    communication buffer, then each of 6 rounds runs one micro-batch while it communicates.  Parameters after every flip must agree."""
     p0 = [1.0, 2.0, 3.0, 4.0]
     lr = 0.1
+    ref_trace = torch.from_numpy(np.load(os.path.join(GOLDEN, "acco_reference_trace.npy")))
+    assert ref_trace.shape == (6, 4) and ref_trace.dtype == torch.float32
 
-    # ---- reference side -------------------------------------------------------------------
-    params = torch.tensor(p0)
-    k = [0]
-
-    def grad_at(p):
-        g = 0.1 * (k[0] + 1) * p
-        k[0] += 1
-        return g
-
-    params.grad = grad_at(params).clone()                       # prepare_grads: g0 at theta0 (kept, not zeroed)
-    com_buffer = params.grad.clone()                             # prepare_buffer_com, no warm-up: grads, count 1
-    count_this_round = torch.ones(1, dtype=torch.int)
-    count_local = torch.ones(1, dtype=torch.int)
-    params_opt = params.clone().float()
-    params_opt.grad = torch.zeros_like(params_opt)
-    opt = torch.optim.AdamW([params_opt], lr=lr, weight_decay=0.0, betas=(0.9, 0.95))
-    sched = torch.optim.lr_scheduler.LambdaLR(opt, lambda s: 1.0)
-    ref_trace = []
-    for r in range(6):
-        ref.communication_step(0, 4, 4, None, count_this_round, com_buffer, params_opt, opt, sched, r)
-        params.grad.add_(grad_at(params))                        # main thread: one micro-batch during the round
-        count_local.add_(1)
-        ref.update_buffers_step(params, com_buffer, 4, count_this_round, count_local, r)
-        ref_trace.append(params.clone())
-
-    # ---- ours -----------------------------------------------------------------------------
     t = make("acco", model=ToyQuadratic(p0), nb_steps_tot=10 ** 6, learning_rate=lr, reference_quirks=True,
              adam_beta1=0.9, adam_beta2=0.95)
     ours = []
